@@ -50,6 +50,27 @@ MAC_PER_TOM_MODMUL = 117   # EXECUTED IMAD.WIDE per 258-bit product: 9 rows x (9
 MAC_PER_P256_MODMUL = 64   # p256.p product scanning: 8 x 8, the reduction is additions only
 MAC_PER_N256_MODMUL = 136  # p256.n generic CIOS: 64 + 64 + 8
 W_PROVE_REF = {8: 6861088, 256: 6942368, 1024: 6974880}   # reference-algorithm modmuls/proof (SURVEY 8(d))
+DUMP_BYTES = 60 << 20      # --dump-outputs: the arrays together; with the .npy headers all files stay below 64 MB
+
+
+def dump_rows(B: int, row_bytes: int, fixed_bytes: int):
+    """Rows of a (B, row_bytes) float32 array that fit in DUMP_BYTES beside `fixed_bytes`: all of them, or a fixed
+    seeded sample in ascending order."""
+    import numpy as np
+    k = max(1, min(B, (DUMP_BYTES - fixed_bytes) // (4 * row_bytes)))
+    return np.arange(B) if k == B else np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+
+
+def dump_outputs(out_dir: str, rows, proofs, proof_len, status, **extra):
+    """Write what one prove call returned as float32 .npy files: the proof bytes of `rows` (zero past each proof's
+    length, where the bytes are padding), every proof length and status, the row indices, and `extra` arrays."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    proofs = np.asarray(proofs).astype(np.float32)
+    proofs[np.arange(proofs.shape[1])[None, :] >= np.asarray(proof_len)[rows][:, None]] = 0
+    arrays = {'proofs': proofs, 'proof_rows': rows, 'proof_len': proof_len, 'status': status, **extra}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a).astype(np.float32))
 
 
 # ----------------------------------------------------------------------------------------- CPU arm
@@ -153,6 +174,10 @@ def run_reference(args):
         smp = port.sample(cores, 4000 + k)      # building the sample (keygen, signatures) is not timed
         tot_s += port.prove(smp)
         tot_n += cores
+    if args.dump_outputs:
+        _, _, _, proofs, plen, st, ps = smp
+        rows = dump_rows(cores, ps, 3 * 4 * cores)
+        dump_outputs(args.dump_outputs, rows, proofs[rows], plen, st)
     v = tot_n / tot_s
     line = {
         'impl': 'reference', 'metric': 'ZKAttest proofs/sec', 'value': v, 'unit': 'proofs/s',
@@ -482,6 +507,12 @@ def run_ours(args):
     ms_total = timed(step_device, args.steps, drain)
     launches = L.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the output buffer set of the last timed step, read before the passes below prove into it again
+        out_p, out_l = outbufs[(step_no[0] - 1) % len(outbufs)]
+        rows = dump_rows(B, ps, 5 * 4 * B)
+        dump = {'proofs': out_p[torch.from_numpy(rows).to(dev)].cpu().numpy(), 'proof_len': out_l.cpu().numpy(),
+                'status': stat_d.cpu().numpy()}
     ms_step = ms_total / args.steps
     value = world * B / (ms_step * 1e-3)
     gather_info = None
@@ -567,6 +598,9 @@ def run_ours(args):
     all_ok = bool((ok_d == 1).all().item()) and bool((vst_d == 0).all().item())
     if world > 1:
         all_ok = all_ok and bool((ok_all == 1).all().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, rows, dump['proofs'], dump['proof_len'], dump['status'],
+                     verify_ok=ok_d.cpu().numpy(), verify_status=vst_d.cpu().numpy())
     L.set_option('lanes', 1)
     L.profile_reset()
     L.set_profiling(True)
@@ -779,7 +813,13 @@ def main():
     ap.add_argument('--batch', type=int, default=0)
     ap.add_argument('--ring', type=int, default=0)
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one returned to DIR/<name>.npy (float32): proofs '
+                         '(a seeded sample of rows when all of them exceed 60 MiB; proof_rows names them), proof_len, '
+                         'status and, for --impl ours, verify_ok / verify_status of the timed verify leg; rank 0 only')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:
